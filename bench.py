@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — training examples/sec of the xflow hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workloads a,b,...] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workloads a,b,...] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch per GPU: LRWorker::update / FMWorker::update (pull,
 forward, gradient, push) plus the server-side FTRL step it triggers.  The line's own numbers are the
@@ -57,6 +57,7 @@ WORKLOADS = {
 }
 MAIN = "headline_lr"
 RING = 8  # distinct batches cycled through (8 x 52 MB of keys > 126 MB L2; the tables are GBs)
+DUMP_KEYS = 1 << 16  # keys per workload written by --dump-outputs: all six workloads stay under 32 MB
 
 
 def load_peaks():
@@ -170,7 +171,6 @@ def cpu_reference(wl, rows, warm_epochs, cores, servers):
                    how="oracle/_ref/xflow_ref = the reference's src/ compiled unmodified (-O2) + in-process ps shim "
                        "(zero transport cost), core_num=%d worker threads, %d key-range server shard(s)" % (cores, servers))
     else:
-        O.build()
         t = O.Table(K=wl["K"], opt=O.OPT_FTRL if wl["opt"] == "ftrl" else O.OPT_SGD)
         t0 = time.perf_counter()
         O.train_file(t, train + "-00000", size_mb << 20, 1)
@@ -312,6 +312,21 @@ def text_leg(api, tr, wl, rank, steps, warm, barrier):
     return out
 
 
+def dump_outputs(out_dir, name, wl, table, d_keys):
+    """What the device-resident timed path computed in its last step: the table rows of that batch's keys as the
+    step left them (what a pull or export returns), on a fixed, seeded sample of DUMP_KEYS of its unique keys in
+    key order.  One float32 file per field, <out_dir>/<workload>.<field>.npy (FM k=16 + FTRL: 13 MB)."""
+    keys = np.unique(d_keys.cpu().numpy().view(np.uint64))
+    keys = keys[np.sort(np.random.default_rng(0).choice(keys.size, min(DUMP_KEYS, keys.size), replace=False))]
+    e = table.export(keys)
+    assert e["present"].all()
+    fields = ["w", "nw", "zw"] if wl["opt"] == "ftrl" else ["w"]
+    if wl["K"]:
+        fields += ["v", "nv", "zv"] if wl["opt"] == "ftrl" else ["v"]
+    for f in fields:
+        np.save(os.path.join(out_dir, "%s.%s.npy" % (name, f)), e[f].astype(np.float32))
+
+
 def run_workload(name, wl, args, rank, world, local, comm, api, torch, stream, sampler, barrier, allmax):
     B, nnz = B_ROWS, B_ROWS * wl["nnz"]
     model = api.MODEL_LR if wl["model"] == "lr" else api.MODEL_FM
@@ -356,6 +371,8 @@ def run_workload(name, wl, args, rank, world, local, comm, api, torch, stream, s
         st1 = tr.stats()
         launches = tr.launches() - l0
         sampler_windows = [(t_w0, t_w1)]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, name, wl, table, ring.dev[(args.warmup + args.steps - 1) % RING][1])
         # ---------------- end-to-end, binary: page-locked host CSR of u32 ids, hashed on the device
         def one(i, addr):
             p = ring.pin[i % RING]
@@ -376,7 +393,7 @@ def run_workload(name, wl, args, rank, world, local, comm, api, torch, stream, s
         # ---------------- end-to-end, text (the headline e2e): what the reference arm does from its shard
         text = None
         if not args.no_text_e2e:
-            text = text_leg(api, tr, wl, rank, max(3, min(args.steps, 20)), 2, barrier)
+            text = text_leg(api, tr, wl, rank, args.steps, 2, barrier)
     ms, ms_bin = allmax(ms), allmax(ms_bin)
     steps = args.steps
     U = (st1["unique_keys"] - st0["unique_keys"]) / max(steps, 1)
@@ -456,7 +473,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-text-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps of each workload, write what its last step computed to DIR (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -471,6 +492,10 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus and world > 1:
         raise SystemExit("--gpus %d but WORLD_SIZE=%d" % (args.gpus, world))
+    if args.dump_outputs:
+        if world > 1:
+            raise SystemExit("--dump-outputs needs a single process: each rank's table holds only its key range")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if api.device_count() < 1:
         raise SystemExit("bench.py needs a CUDA device: the product has no CPU path")
     torch.cuda.set_device(local)

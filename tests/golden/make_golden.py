@@ -8,6 +8,7 @@ reference's final table (w and, for FTRL, n and z; v rows for FM), the initial t
 replays a pre-initialised latent table, the reference's predictions (as printed to pred_0_0.txt,
 6 significant digits) and its logloss / auc line.  The synthetic text inputs are regenerated from a
 seed by xflow_b200.datagen (bit-reproducible), the bundled 200-row shards are copied as data fixtures.
+Each REF_RUNS entry is stored as the reference's final table on a sample of its keys.
 """
 import os
 import shutil
@@ -25,7 +26,24 @@ from xflow_b200 import datagen  # noqa: E402
 
 REF_DATA = "/root/reference/data"
 
-from cases import CASES, SYN, SYN_TEST  # noqa: E402
+from cases import CASES, REF_RUNS, SYN, SYN_TEST, ref_run_name  # noqa: E402
+
+
+def sample_rows(n, size):
+    """A fixed, seeded choice of `size` of `n` rows, sorted."""
+    return np.sort(np.random.default_rng(0).choice(n, size, replace=False))
+
+
+def ref_run_keys(keys, train_prefix, size=512, hot=32):
+    """Of a reference run's sorted `keys`, the ones stored: the `hot` most frequent keys of the training shard
+    (the keys whose many occurrences per batch the reference sums in float32) and a seeded sample of the rest,
+    `size` in all.  Returns a boolean mask over `keys`."""
+    seen = np.concatenate([k for _, k, _ in O.load_blocks(train_prefix + "-00000", 1 << 20)])
+    uk, cnt = np.unique(seen, return_counts=True)
+    mask = np.isin(keys, uk[np.argsort(-cnt, kind="stable")[:hot]])
+    rest = np.flatnonzero(~mask)
+    mask[rest[sample_rows(rest.size, size - int(mask.sum()))]] = True
+    return mask
 
 
 def materialise_data(kind, tmp):
@@ -68,11 +86,26 @@ def main():
             assert np.array_equal(p["keys"], d["keys"])
             out["init_w"] = p["w"]
             out["init_v"] = p["v"]
+        if c.get("latent_rows"):
+            out["latent_rows"] = sample_rows(d["keys"].size, c["latent_rows"])
+            for k in ("v", "nv", "zv"):
+                out[k] = out[k][out["latent_rows"]]
         pred = np.loadtxt(r["pred_path"], ndmin=2)
         out["pred_pctr"] = pred[:, 0].astype(np.float64)
         out["pred_label"] = pred[:, 2].astype(np.int32)
         np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
         print("%-24s keys=%d logloss=%s auc=%s" % (name, d["keys"].size, r["logloss"], r.get("auc")))
+    for model, opt, K, epochs in REF_RUNS:
+        train, test = materialise_data("syn", tmp)
+        run = tempfile.mkdtemp()
+        O.run_ref(model, opt, train, test, epochs, run, core=1, block_mb=1, vdim=K or 10,
+                  dump=os.path.join(run, "final.bin"), fix_time=1.5e9)
+        d = O.read_dump(os.path.join(run, "final.bin"))
+        keep = ref_run_keys(d["keys"], train)
+        name = ref_run_name(model, opt, K, epochs)
+        np.savez_compressed(os.path.join(HERE, name + ".npz"),
+                            **{k: d[k][keep] for k in ("keys", "w", "nw", "zw", "v", "nv", "zv") if k in d})
+        print("%-24s keys=%d of %d" % (name, int(keep.sum()), d["keys"].size))
     # known-answer vectors of std::hash<std::string> (libstdc++), via the real std::hash
     strs = [b"0", b"1163", b"8672", b"185", b"7755", b"", b"1520", b"2738", b"123456789",
             b"feature_with_a_long_name_0123456789"]

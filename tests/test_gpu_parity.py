@@ -10,7 +10,8 @@ import numpy as np
 import pytest
 
 from cases import CASES
-from common import check_fm_first_step, assert_close, assert_close_noise_aware, data_prefixes, golden, oracle_case_run
+from common import (check_fm_first_step, assert_close, assert_close_noise_aware, data_prefixes, golden, oracle_case_run,
+                    stored_rows)
 from oracle import oracle as O
 from xflow_b200 import api, datagen
 
@@ -64,7 +65,8 @@ def test_golden_case_matches_reference(case, syn_data):
         x, _, xp = oracle_case_run(case, syn_data, exact=True)
         for k in ("w", "nw", "zw", "v", "nv", "zv"):
             if k in g.files:
-                assert_close_noise_aware(e[k], g[k], x[k], "%s.%s" % (case, k), max_noisy_frac=0.02)
+                assert_close_noise_aware(stored_rows(e, g, k), g[k], stored_rows(x, g, k), "%s.%s" % (case, k),
+                                         max_noisy_frac=0.02)
         # a single noisy hot key shows in every row that contains it: no bound on the noisy fraction
         assert_close_noise_aware(p, g["pred_pctr"], xp, case + ".pctr", rel=2e-5, abs_floor=6e-7,
                                  max_noisy_frac=1.0)
@@ -86,7 +88,7 @@ def test_golden_case_with_table_growth(syn_data):
     assert table.capacity() >= 2 * g["keys"].size
     x, _, _ = oracle_case_run(case, syn_data, exact=True)
     for k in ("w", "nw", "zw", "v", "nv", "zv"):
-        assert_close_noise_aware(e[k], g[k], x[k], "growth.%s" % k, max_noisy_frac=0.02)
+        assert_close_noise_aware(stored_rows(e, g, k), g[k], stored_rows(x, g, k), "growth.%s" % k, max_noisy_frac=0.02)
 
 
 @pytest.mark.parametrize("model,opt,K", [("lr", "ftrl", 0), ("lr", "sgd", 0), ("fm", "sgd", 8), ("fm", "ftrl", 16),
