@@ -773,17 +773,35 @@ static int xf_check_batch(xf_trainer* tr, uint32_t rows, uint32_t nnz) {
   return XF_OK;
 }
 
-// the step proper, on device-resident CSR; mode 0 = train, 1 = predict
-static int xf_step_device_impl(xf_trainer* tr, const uint32_t* d_row_ptr, const uint64_t* d_keys,
-                               const uint8_t* d_labels, uint32_t rows, uint32_t nnz, int mode, float* d_abs,
-                               const float* d_vals = nullptr, const uint8_t* d_fields = nullptr) {
+// One batch as the step kernels read it: CSR arrays (keys, or u32 ids that are hashed to keys on the device), the
+// canonical FM's feature values and the multi-view machine's field ids.  Host or device pointers, as the user says.
+struct XfBatch {
+  const uint32_t* row_ptr = nullptr;
+  const uint64_t* keys = nullptr;
+  const uint8_t* labels = nullptr;
+  uint32_t rows = 0, nnz = 0;
+  const float* vals = nullptr;
+  const uint8_t* fields = nullptr;
+  const uint32_t* ids = nullptr;
+};
+
+static void xf_count_step(xf_trainer* tr, uint32_t rows, uint32_t nnz) {
+  ++tr->n_steps;
+  tr->n_rows += rows;
+  tr->n_nnz += nnz;
+  tr->last_rows = rows;
+}
+
+// the step proper, on a device-resident batch; mode 0 = train, 1 = predict
+static int xf_step_device_impl(xf_trainer* tr, const XfBatch& d, int mode, float* d_abs) {
   xf_table* t = tr->table;
+  const uint32_t rows = d.rows, nnz = d.nnz;
   if (rows == 0 && !tr->mg) return XF_OK;     // sharded: an empty batch still takes part in the exchange
   if (!tr->mg) XF_TRY(t->ensure_room(nnz));  // the sharded path sizes the shard from what it receives
   cudaStream_t st = t->stream;
   const bool prof = tr->profile && mode == 0;
   cudaEvent_t* pe = nullptr;
-  if (tr->mg && !prof) return xf_mg_step(tr, d_row_ptr, d_keys, d_labels, rows, nnz, mode, d_abs, nullptr);
+  if (tr->mg && !prof) return xf_mg_step(tr, d.row_ptr, d.keys, d.labels, rows, nnz, mode, d_abs, nullptr);
   if (prof) {
     if (tr->prof_used + 4 > tr->prof_events.size()) {
       size_t old = tr->prof_events.size();
@@ -792,15 +810,17 @@ static int xf_step_device_impl(xf_trainer* tr, const uint32_t* d_row_ptr, const 
     }
     pe = &tr->prof_events[tr->prof_used];
     tr->prof_used += 4;
-    if (tr->mg) return xf_mg_step(tr, d_row_ptr, d_keys, d_labels, rows, nnz, mode, d_abs, pe);
+    if (tr->mg) return xf_mg_step(tr, d.row_ptr, d.keys, d.labels, rows, nnz, mode, d_abs, pe);
     XF_CUDA_TRY(cudaEventRecord(pe[0], st));
   }
+  // per-row outputs: the residuals when the trainer keeps them, the predictions of a forward pass
+  float* loss = (mode == 0 && tr->cfg.keep_loss) ? tr->loss.as<float>() : nullptr;
+  float* pctr = mode == 1 ? tr->pctr.as<float>() : nullptr;
   if (t->view.lazy) {
     // one kernel: the optimizer step of earlier batches is folded in as rows are touched
     if (mode == 0) XF_TRY(t->next_seq());
-    xf_launch_step_lr_lazy(t->view, d_row_ptr, d_keys, d_labels, (int)rows, mode, t->seq, t->d_rows_by_seq,
-                           (mode == 0 && tr->cfg.keep_loss) ? tr->loss.as<float>() : nullptr,
-                           mode == 1 ? tr->pctr.as<float>() : nullptr, d_abs, tr->d_unique_total, st);
+    xf_launch_step_lr_lazy(t->view, d.row_ptr, d.keys, d.labels, (int)rows, mode, t->seq, t->d_rows_by_seq, loss, pctr,
+                           d_abs, tr->d_unique_total, st);
     ++tr->launches;
     if (prof) {
       XF_CUDA_TRY(cudaEventRecord(pe[1], st));
@@ -812,21 +832,18 @@ static int xf_step_device_impl(xf_trainer* tr, const uint32_t* d_row_ptr, const 
   }
   const bool mvm = tr->cfg.model == XF_MODEL_MVM;
   const bool canon = tr->cfg.model == XF_MODEL_FM_CANONICAL || mvm;
-  if (mvm && !d_fields && nnz) { xf_set_error("XF_MODEL_MVM steps need the tokens' field ids (xf_trainer_step_host_fields)"); return XF_ERR_ARG; }
+  if (mvm && !d.fields && nnz) { xf_set_error("XF_MODEL_MVM steps need the tokens' field ids (xf_trainer_step_host_fields)"); return XF_ERR_ARG; }
   const uint32_t extra = canon ? 0u : xf_step_touched_extra(t->view.K, (int)rows);
   XF_TRY(tr->touched.ensure(((size_t)nnz + extra) * 4));
   if (mvm)
-    xf_launch_step_mvm(t->view, d_row_ptr, d_keys, d_fields, d_vals, d_labels, (int)rows, mode, tr->touched.as<uint32_t>(),
-                       (mode == 0 && tr->cfg.keep_loss) ? tr->loss.as<float>() : nullptr,
-                       mode == 1 ? tr->pctr.as<float>() : nullptr, d_abs, st);
+    xf_launch_step_mvm(t->view, d.row_ptr, d.keys, d.fields, d.vals, d.labels, (int)rows, mode, tr->touched.as<uint32_t>(),
+                       loss, pctr, d_abs, st);
   else if (canon)
-    xf_launch_step_fmc(t->view, d_row_ptr, d_keys, d_vals, d_labels, (int)rows, mode, tr->touched.as<uint32_t>(),
-                       (mode == 0 && tr->cfg.keep_loss) ? tr->loss.as<float>() : nullptr,
-                       mode == 1 ? tr->pctr.as<float>() : nullptr, d_abs, st);
+    xf_launch_step_fmc(t->view, d.row_ptr, d.keys, d.vals, d.labels, (int)rows, mode, tr->touched.as<uint32_t>(), loss,
+                       pctr, d_abs, st);
   else
-    xf_launch_step(t->view, d_row_ptr, d_keys, d_labels, (int)rows, mode, tr->touched.as<uint32_t>(), nnz,
-                   (mode == 0 && tr->cfg.keep_loss) ? tr->loss.as<float>() : nullptr,
-                   mode == 1 ? tr->pctr.as<float>() : nullptr, d_abs, st);
+    xf_launch_step(t->view, d.row_ptr, d.keys, d.labels, (int)rows, mode, tr->touched.as<uint32_t>(), nnz, loss, pctr,
+                   d_abs, st);
   ++tr->launches;
   if (prof) {
     XF_CUDA_TRY(cudaEventRecord(pe[1], st));
@@ -843,15 +860,12 @@ static int xf_step_device_impl(xf_trainer* tr, const uint32_t* d_row_ptr, const 
   return XF_OK;
 }
 
-XF_DLL int xf_trainer_step_device(xf_trainer* tr, const uint32_t* d_row_ptr, const uint64_t* d_keys,
-                                  const uint8_t* d_labels, uint32_t rows, uint32_t nnz) {
-  if (!tr || !d_row_ptr || !d_keys || !d_labels) return XF_ERR_ARG;
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  XF_TRY(xf_step_device_impl(tr, d_row_ptr, d_keys, d_labels, rows, nnz, 0, nullptr));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
+// A training step on a batch the caller keeps on the device: nothing to upload, so no buffer set, no cudaSetDevice
+// and no `consumed` event.  An empty batch is counted as a step.
+static int xf_step_resident(xf_trainer* tr, const XfBatch& d) {
+  XF_TRY(xf_check_batch(tr, d.rows, d.nnz));
+  XF_TRY(xf_step_device_impl(tr, d, 0, nullptr));
+  xf_count_step(tr, d.rows, d.nnz);
   return XF_OK;
 }
 
@@ -866,12 +880,11 @@ static bool xf_is_pinned(const void* p) {
 
 // stage one host array into buffer set `b` (pinned source: DMA directly; pageable: copy through the
 // set's pinned staging) and enqueue the H2D on the copy stream
-static int xf_stage(xf_trainer* tr, XfDevBuf& dev, XfPinBuf& pin, const void* src, size_t bytes, bool staging_free) {
+static int xf_stage(xf_trainer* tr, XfDevBuf& dev, XfPinBuf& pin, const void* src, size_t bytes) {
   if (bytes == 0) return XF_OK;
   XF_TRY(dev.ensure(bytes));
   const void* from = src;
   if (!xf_is_pinned(src)) {
-    (void)staging_free;
     XF_TRY(pin.ensure(bytes));
     memcpy(pin.p, src, bytes);
     from = pin.p;
@@ -880,68 +893,114 @@ static int xf_stage(xf_trainer* tr, XfDevBuf& dev, XfPinBuf& pin, const void* sr
   return XF_OK;
 }
 
-static int xf_upload_batch(xf_trainer* tr, XfBatchBuf& b, const uint32_t* row_ptr, const uint64_t* keys,
-                           const uint8_t* labels, uint32_t rows, uint32_t nnz) {
+// Uploads host batch `h` into buffer set `b` and describes the device copy in *d.  Keys (and labels) go through
+// xf_stage on the copy stream; u32 ids come from page-locked memory, are copied directly and hashed to keys on the
+// copy stream (4 B/token instead of 8 B); values and field ids are plain copies on the table stream (a small part of
+// a batch).  Field ids the MVM kernel has no room for are refused here, before any kernel runs.
+static int xf_upload(xf_trainer* tr, XfBatchBuf& b, const XfBatch& h, XfBatch* d) {
+  const size_t rp_bytes = ((size_t)h.rows + 1) * 4;
   // the device buffers of this set may still be read by the step issued two calls ago
   XF_CUDA_TRY(cudaStreamWaitEvent(tr->copy_stream, b.consumed, 0));
-  // its pinned staging may still be the source of that step's H2D
-  XF_CUDA_TRY(cudaEventSynchronize(b.staged));
-  XF_TRY(xf_stage(tr, b.row_ptr, b.h_row_ptr, row_ptr, ((size_t)rows + 1) * 4, true));
-  XF_TRY(xf_stage(tr, b.keys, b.h_keys, keys, (size_t)nnz * 8, true));
-  if (labels) XF_TRY(xf_stage(tr, b.labels, b.h_labels, labels, (size_t)rows, true));
-  XF_CUDA_TRY(cudaEventRecord(b.staged, tr->copy_stream));
+  if (h.ids) {
+    XF_TRY(b.row_ptr.ensure(rp_bytes));
+    XF_TRY(b.ids.ensure((size_t)h.nnz * 4));
+    XF_TRY(b.keys.ensure((size_t)h.nnz * 8));
+    XF_TRY(b.labels.ensure(h.rows));
+    XF_CUDA_TRY(cudaMemcpyAsync(b.row_ptr.p, h.row_ptr, rp_bytes, cudaMemcpyHostToDevice, tr->copy_stream));
+    XF_CUDA_TRY(cudaMemcpyAsync(b.ids.p, h.ids, (size_t)h.nnz * 4, cudaMemcpyHostToDevice, tr->copy_stream));
+    XF_CUDA_TRY(cudaMemcpyAsync(b.labels.p, h.labels, h.rows, cudaMemcpyHostToDevice, tr->copy_stream));
+    XF_TRY(xf_launch_hash_ids(b.ids.as<uint32_t>(), h.nnz, b.keys.as<uint64_t>(), tr->copy_stream));
+    ++tr->launches;
+  } else {
+    // its pinned staging may still be the source of that step's H2D
+    XF_CUDA_TRY(cudaEventSynchronize(b.staged));
+    XF_TRY(xf_stage(tr, b.row_ptr, b.h_row_ptr, h.row_ptr, rp_bytes));
+    XF_TRY(xf_stage(tr, b.keys, b.h_keys, h.keys, (size_t)h.nnz * 8));
+    if (h.labels) XF_TRY(xf_stage(tr, b.labels, b.h_labels, h.labels, (size_t)h.rows));
+    XF_CUDA_TRY(cudaEventRecord(b.staged, tr->copy_stream));
+  }
   XF_CUDA_TRY(cudaEventRecord(b.copied, tr->copy_stream));
   XF_CUDA_TRY(cudaStreamWaitEvent(tr->table->stream, b.copied, 0));
   tr->input_ready = b.copied;  // the sharded path starts its dedup on another stream
+  if (!h.labels) XF_TRY(b.labels.ensure((size_t)h.rows + 1));  // unused by mode 1 but must be a valid pointer
+  *d = XfBatch{b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), h.rows, h.nnz};
+  if (h.vals && h.nnz) {
+    XF_TRY(b.vals.ensure((size_t)h.nnz * 4));
+    XF_CUDA_TRY(cudaMemcpyAsync(b.vals.p, h.vals, (size_t)h.nnz * 4, cudaMemcpyHostToDevice, tr->table->stream));
+    d->vals = b.vals.as<float>();
+  }
+  if (h.fields && h.nnz) {
+    for (uint32_t j = 0; j < h.nnz; ++j)
+      if (h.fields[j] >= XF_MVM_FIELDS) { xf_set_error("field id %u of token %u: XF_MODEL_MVM takes field ids below %d", (unsigned)h.fields[j], j, XF_MVM_FIELDS); return XF_ERR_ARG; }
+    XF_TRY(b.fields.ensure((size_t)h.nnz));
+    XF_CUDA_TRY(cudaMemcpyAsync(b.fields.p, h.fields, (size_t)h.nnz, cudaMemcpyHostToDevice, tr->table->stream));
+    d->fields = b.fields.as<uint8_t>();
+  }
   return XF_OK;
+}
+
+// What an entry point that takes a host batch hands back once the step is enqueued.
+struct XfHostReturn {
+  enum { NO_WAIT, WAIT, WAIT_CHECKED } wait;  // synchronise on the table stream (and check the table's error word)
+  float* mean_abs_loss;      // mode 0, after the wait: the mean |loss| of the batch (0 for an empty batch)
+  float* pctr_out;           // mode 1: the predictions, copied before the wait
+  float* pinned_loss_sum;    // mode 0, no wait: the loss sum, copied asynchronously into this page-locked float
+  const char* page_locked;   // the entry point's name if every host array must be page-locked
+};
+
+// A host batch through one of the two buffer sets: upload, step, release the set, count, read back.
+static int xf_step_host_batch(xf_trainer* tr, const XfBatch& h, int mode, const XfHostReturn& r) {
+  XF_TRY(xf_check_batch(tr, h.rows, h.nnz));
+  if (h.rows == 0 && !tr->mg) {
+    if (r.mean_abs_loss) *r.mean_abs_loss = 0.f;
+    return XF_OK;
+  }
+  if (r.page_locked && (!xf_is_pinned(h.row_ptr) || !xf_is_pinned(h.ids ? (const void*)h.ids : h.keys) ||
+                        !xf_is_pinned(h.labels) || (r.pinned_loss_sum && !xf_is_pinned(r.pinned_loss_sum)))) {
+    xf_set_error("%s needs page-locked host buffers", r.page_locked);
+    return XF_ERR_ARG;
+  }
+  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
+  const int slot = (int)(tr->step_index & 1);
+  XfBatchBuf& b = tr->buf[slot];
+  ++tr->step_index;
+  XfBatch d;
+  XF_TRY(xf_upload(tr, b, h, &d));
+  cudaStream_t st = tr->table->stream;
+  float* d_abs = mode == 0 ? tr->d_abs_loss + slot : nullptr;
+  if (d_abs) XF_CUDA_TRY(cudaMemsetAsync(d_abs, 0, sizeof(float), st));
+  XF_TRY(xf_step_device_impl(tr, d, mode, d_abs));
+  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
+  if (mode == 0) xf_count_step(tr, h.rows, h.nnz);
+  if (r.pinned_loss_sum)
+    XF_CUDA_TRY(cudaMemcpyAsync(r.pinned_loss_sum, d_abs, sizeof(float), cudaMemcpyDeviceToHost, st));
+  if (r.wait == XfHostReturn::NO_WAIT) return XF_OK;
+  if (mode == 0)
+    XF_CUDA_TRY(cudaMemcpyAsync(tr->h_abs_loss + slot, d_abs, sizeof(float), cudaMemcpyDeviceToHost, st));
+  else
+    XF_CUDA_TRY(cudaMemcpyAsync(r.pctr_out, tr->pctr.p, (size_t)h.rows * 4, cudaMemcpyDeviceToHost, st));
+  XF_CUDA_TRY(cudaStreamSynchronize(st));  // also: the caller may reuse its arrays (values, field ids) now
+  if (r.mean_abs_loss) *r.mean_abs_loss = h.rows ? tr->h_abs_loss[slot] / (float)h.rows : 0.f;
+  return r.wait == XfHostReturn::WAIT_CHECKED ? tr->table->check_error() : XF_OK;
+}
+
+XF_DLL int xf_trainer_step_device(xf_trainer* tr, const uint32_t* d_row_ptr, const uint64_t* d_keys,
+                                  const uint8_t* d_labels, uint32_t rows, uint32_t nnz) {
+  if (!tr || !d_row_ptr || !d_keys || !d_labels) return XF_ERR_ARG;
+  return xf_step_resident(tr, {d_row_ptr, d_keys, d_labels, rows, nnz});
 }
 
 XF_DLL int xf_trainer_step_host(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys,
                                 const uint8_t* labels, uint32_t rows, uint32_t nnz, float* mean_abs_loss) {
   if (!tr || !row_ptr || (!keys && nnz) || !labels) return XF_ERR_ARG;
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0 && !tr->mg) { if (mean_abs_loss) *mean_abs_loss = 0.f; return XF_OK; }
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, labels, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  XF_CUDA_TRY(cudaMemsetAsync(tr->d_abs_loss + slot, 0, sizeof(float), st));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows,
-                             nnz, 0, tr->d_abs_loss + slot));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  if (mean_abs_loss) {
-    XF_CUDA_TRY(cudaMemcpyAsync(tr->h_abs_loss + slot, tr->d_abs_loss + slot, sizeof(float),
-                                cudaMemcpyDeviceToHost, st));
-    XF_CUDA_TRY(cudaStreamSynchronize(st));
-    *mean_abs_loss = rows ? tr->h_abs_loss[slot] / (float)rows : 0.f;
-  }
-  return XF_OK;
+  return xf_step_host_batch(tr, {row_ptr, keys, labels, rows, nnz}, 0,
+                            {mean_abs_loss ? XfHostReturn::WAIT : XfHostReturn::NO_WAIT, mean_abs_loss});
 }
 
 XF_DLL int xf_trainer_predict_host(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys, uint32_t rows,
                                    uint32_t nnz, float* pctr_out) {
   if (!tr || !row_ptr || (!keys && nnz) || !pctr_out) return XF_ERR_ARG;
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0 && !tr->mg) return XF_OK;
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, nullptr, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  XF_TRY(b.labels.ensure((size_t)rows + 1));  // unused by mode 1 but must be a valid pointer
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows,
-                             nnz, 1, nullptr));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaStreamSynchronize(st));
-  return tr->table->check_error();
+  return xf_step_host_batch(tr, {row_ptr, keys, nullptr, rows, nnz}, 1, {XfHostReturn::WAIT_CHECKED, nullptr, pctr_out});
 }
 
 // ---- the same entry points with feature values (XF_MODEL_FM_CANONICAL, step_fmc.cu)
@@ -949,117 +1008,32 @@ XF_DLL int xf_trainer_step_device_values(xf_trainer* tr, const uint32_t* d_row_p
                                          const float* d_vals, const uint8_t* d_labels, uint32_t rows, uint32_t nnz) {
   if (!tr || !d_row_ptr || !d_keys || !d_labels) return XF_ERR_ARG;
   if (tr->cfg.model != XF_MODEL_FM_CANONICAL) { xf_set_error("feature values need XF_MODEL_FM_CANONICAL"); return XF_ERR_ARG; }
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  XF_TRY(xf_step_device_impl(tr, d_row_ptr, d_keys, d_labels, rows, nnz, 0, nullptr, d_vals));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  return XF_OK;
-}
-
-static int xf_upload_vals(xf_trainer* tr, XfBatchBuf& b, const float* vals, uint32_t nnz, const float** d_vals) {
-  *d_vals = nullptr;
-  if (!vals || !nnz) return XF_OK;
-  XF_TRY(b.vals.ensure((size_t)nnz * 4));
-  // pageable or pinned: a plain stream-ordered copy on the table stream (the values are a small part of a batch)
-  XF_CUDA_TRY(cudaMemcpyAsync(b.vals.p, vals, (size_t)nnz * 4, cudaMemcpyHostToDevice, tr->table->stream));
-  *d_vals = b.vals.as<float>();
-  return XF_OK;
+  return xf_step_resident(tr, {d_row_ptr, d_keys, d_labels, rows, nnz, d_vals});
 }
 
 XF_DLL int xf_trainer_step_host_values(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys, const float* vals,
                                        const uint8_t* labels, uint32_t rows, uint32_t nnz, float* mean_abs_loss) {
   if (!tr || !row_ptr || (!keys && nnz) || !labels) return XF_ERR_ARG;
   if (tr->cfg.model != XF_MODEL_FM_CANONICAL) { xf_set_error("feature values need XF_MODEL_FM_CANONICAL"); return XF_ERR_ARG; }
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0) { if (mean_abs_loss) *mean_abs_loss = 0.f; return XF_OK; }
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, labels, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  const float* d_vals = nullptr;
-  XF_TRY(xf_upload_vals(tr, b, vals, nnz, &d_vals));
-  XF_CUDA_TRY(cudaMemsetAsync(tr->d_abs_loss + slot, 0, sizeof(float), st));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows, nnz, 0,
-                             tr->d_abs_loss + slot, d_vals));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  XF_CUDA_TRY(cudaMemcpyAsync(tr->h_abs_loss + slot, tr->d_abs_loss + slot, sizeof(float), cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaStreamSynchronize(st));  // also: `vals` may be reused by the caller
-  if (mean_abs_loss) *mean_abs_loss = tr->h_abs_loss[slot] / (float)rows;
-  return tr->table->check_error();
+  return xf_step_host_batch(tr, {row_ptr, keys, labels, rows, nnz, vals}, 0, {XfHostReturn::WAIT_CHECKED, mean_abs_loss});
 }
 
 XF_DLL int xf_trainer_predict_host_values(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys, const float* vals,
                                           uint32_t rows, uint32_t nnz, float* pctr_out) {
   if (!tr || !row_ptr || (!keys && nnz) || !pctr_out) return XF_ERR_ARG;
   if (tr->cfg.model != XF_MODEL_FM_CANONICAL) { xf_set_error("feature values need XF_MODEL_FM_CANONICAL"); return XF_ERR_ARG; }
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0) return XF_OK;
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, nullptr, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  XF_TRY(b.labels.ensure((size_t)rows + 1));
-  const float* d_vals = nullptr;
-  XF_TRY(xf_upload_vals(tr, b, vals, nnz, &d_vals));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows, nnz, 1,
-                             nullptr, d_vals));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaStreamSynchronize(st));
-  return tr->table->check_error();
+  return xf_step_host_batch(tr, {row_ptr, keys, nullptr, rows, nnz, vals}, 1,
+                            {XfHostReturn::WAIT_CHECKED, nullptr, pctr_out});
 }
 
 // ---- the defined multi-view machine (XF_MODEL_MVM, step_mvm.cu): the batch with the tokens' field ids
-static int xf_upload_fields(xf_trainer* tr, XfBatchBuf& b, const uint8_t* fields, uint32_t nnz, const uint8_t** d_fields) {
-  *d_fields = nullptr;
-  if (!nnz) return XF_OK;
-  for (uint32_t j = 0; j < nnz; ++j)
-    if (fields[j] >= XF_MVM_FIELDS) { xf_set_error("field id %u of token %u: XF_MODEL_MVM takes field ids below %d", (unsigned)fields[j], j, XF_MVM_FIELDS); return XF_ERR_ARG; }
-  XF_TRY(b.fields.ensure((size_t)nnz));
-  XF_CUDA_TRY(cudaMemcpyAsync(b.fields.p, fields, (size_t)nnz, cudaMemcpyHostToDevice, tr->table->stream));
-  *d_fields = b.fields.as<uint8_t>();
-  return XF_OK;
-}
-
 XF_DLL int xf_trainer_step_host_fields(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys, const uint8_t* fields,
                                        const float* vals, const uint8_t* labels, uint32_t rows, uint32_t nnz,
                                        float* mean_abs_loss) {
   if (!tr || !row_ptr || (!keys && nnz) || (!fields && nnz) || !labels) return XF_ERR_ARG;
   if (tr->cfg.model != XF_MODEL_MVM) { xf_set_error("field ids need XF_MODEL_MVM"); return XF_ERR_ARG; }
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0) { if (mean_abs_loss) *mean_abs_loss = 0.f; return XF_OK; }
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, labels, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  const float* d_vals = nullptr;
-  const uint8_t* d_fields = nullptr;
-  XF_TRY(xf_upload_vals(tr, b, vals, nnz, &d_vals));
-  XF_TRY(xf_upload_fields(tr, b, fields, nnz, &d_fields));
-  XF_CUDA_TRY(cudaMemsetAsync(tr->d_abs_loss + slot, 0, sizeof(float), st));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows, nnz, 0,
-                             tr->d_abs_loss + slot, d_vals, d_fields));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  XF_CUDA_TRY(cudaMemcpyAsync(tr->h_abs_loss + slot, tr->d_abs_loss + slot, sizeof(float), cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaStreamSynchronize(st));  // also: `fields` / `vals` may be reused by the caller
-  if (mean_abs_loss) *mean_abs_loss = tr->h_abs_loss[slot] / (float)rows;
-  return tr->table->check_error();
+  return xf_step_host_batch(tr, {row_ptr, keys, labels, rows, nnz, vals, fields}, 0,
+                            {XfHostReturn::WAIT_CHECKED, mean_abs_loss});
 }
 
 XF_DLL int xf_trainer_predict_host_fields(xf_trainer* tr, const uint32_t* row_ptr, const uint64_t* keys,
@@ -1067,25 +1041,8 @@ XF_DLL int xf_trainer_predict_host_fields(xf_trainer* tr, const uint32_t* row_pt
                                           float* pctr_out) {
   if (!tr || !row_ptr || (!keys && nnz) || (!fields && nnz) || !pctr_out) return XF_ERR_ARG;
   if (tr->cfg.model != XF_MODEL_MVM) { xf_set_error("field ids need XF_MODEL_MVM"); return XF_ERR_ARG; }
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0) return XF_OK;
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, nullptr, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  XF_TRY(b.labels.ensure((size_t)rows + 1));
-  const float* d_vals = nullptr;
-  const uint8_t* d_fields = nullptr;
-  XF_TRY(xf_upload_vals(tr, b, vals, nnz, &d_vals));
-  XF_TRY(xf_upload_fields(tr, b, fields, nnz, &d_fields));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows, nnz, 1,
-                             nullptr, d_vals, d_fields));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaStreamSynchronize(st));
-  return tr->table->check_error();
+  return xf_step_host_batch(tr, {row_ptr, keys, nullptr, rows, nnz, vals, fields}, 1,
+                            {XfHostReturn::WAIT_CHECKED, nullptr, pctr_out});
 }
 
 XF_DLL int xf_trainer_init_push(xf_trainer* tr) {
@@ -1149,73 +1106,18 @@ XF_DLL int xf_trainer_step_host_async(xf_trainer* tr, const uint32_t* row_ptr, c
                                       const uint8_t* labels, uint32_t rows, uint32_t nnz,
                                       float* pinned_abs_loss_sum) {
   if (!tr || !row_ptr || (!keys && nnz) || !labels) return XF_ERR_ARG;
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0 && !tr->mg) return XF_OK;
-  if (!xf_is_pinned(row_ptr) || !xf_is_pinned(keys) || !xf_is_pinned(labels) ||
-      (pinned_abs_loss_sum && !xf_is_pinned(pinned_abs_loss_sum))) {
-    xf_set_error("xf_trainer_step_host_async needs page-locked host buffers");
-    return XF_ERR_ARG;
-  }
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  XF_TRY(xf_upload_batch(tr, b, row_ptr, keys, labels, rows, nnz));
-  cudaStream_t st = tr->table->stream;
-  XF_CUDA_TRY(cudaMemsetAsync(tr->d_abs_loss + slot, 0, sizeof(float), st));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows,
-                             nnz, 0, tr->d_abs_loss + slot));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  if (pinned_abs_loss_sum)
-    XF_CUDA_TRY(cudaMemcpyAsync(pinned_abs_loss_sum, tr->d_abs_loss + slot, sizeof(float), cudaMemcpyDeviceToHost, st));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  return XF_OK;
+  return xf_step_host_batch(tr, {row_ptr, keys, labels, rows, nnz}, 0,
+                            {XfHostReturn::NO_WAIT, nullptr, nullptr, pinned_abs_loss_sum, "xf_trainer_step_host_async"});
 }
 
 XF_DLL int xf_trainer_step_host_ids_async(xf_trainer* tr, const uint32_t* row_ptr, const uint32_t* ids,
                                           const uint8_t* labels, uint32_t rows, uint32_t nnz,
                                           float* pinned_abs_loss_sum) {
   if (!tr || !row_ptr || (!ids && nnz) || !labels) return XF_ERR_ARG;
-  XF_TRY(xf_check_batch(tr, rows, nnz));
-  if (rows == 0 && !tr->mg) return XF_OK;
-  if (!xf_is_pinned(row_ptr) || !xf_is_pinned(ids) || !xf_is_pinned(labels) ||
-      (pinned_abs_loss_sum && !xf_is_pinned(pinned_abs_loss_sum))) {
-    xf_set_error("xf_trainer_step_host_ids_async needs page-locked host buffers");
-    return XF_ERR_ARG;
-  }
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  const int slot = (int)(tr->step_index & 1);
-  XfBatchBuf& b = tr->buf[slot];
-  ++tr->step_index;
-  // upload row_ptr, ids (4 B/token instead of 8 B keys) and labels; hash on the device
-  XF_CUDA_TRY(cudaStreamWaitEvent(tr->copy_stream, b.consumed, 0));
-  XF_TRY(b.row_ptr.ensure(((size_t)rows + 1) * 4));
-  XF_TRY(b.ids.ensure((size_t)nnz * 4));
-  XF_TRY(b.keys.ensure((size_t)nnz * 8));
-  XF_TRY(b.labels.ensure(rows));
-  XF_CUDA_TRY(cudaMemcpyAsync(b.row_ptr.p, row_ptr, ((size_t)rows + 1) * 4, cudaMemcpyHostToDevice, tr->copy_stream));
-  XF_CUDA_TRY(cudaMemcpyAsync(b.ids.p, ids, (size_t)nnz * 4, cudaMemcpyHostToDevice, tr->copy_stream));
-  XF_CUDA_TRY(cudaMemcpyAsync(b.labels.p, labels, rows, cudaMemcpyHostToDevice, tr->copy_stream));
-  XF_TRY(xf_launch_hash_ids(b.ids.as<uint32_t>(), nnz, b.keys.as<uint64_t>(), tr->copy_stream));
-  ++tr->launches;
-  XF_CUDA_TRY(cudaEventRecord(b.copied, tr->copy_stream));
-  cudaStream_t st = tr->table->stream;
-  XF_CUDA_TRY(cudaStreamWaitEvent(st, b.copied, 0));
-  tr->input_ready = b.copied;
-  XF_CUDA_TRY(cudaMemsetAsync(tr->d_abs_loss + slot, 0, sizeof(float), st));
-  XF_TRY(xf_step_device_impl(tr, b.row_ptr.as<uint32_t>(), b.keys.as<uint64_t>(), b.labels.as<uint8_t>(), rows,
-                             nnz, 0, tr->d_abs_loss + slot));
-  XF_CUDA_TRY(cudaEventRecord(b.consumed, st));
-  if (pinned_abs_loss_sum)
-    XF_CUDA_TRY(cudaMemcpyAsync(pinned_abs_loss_sum, tr->d_abs_loss + slot, sizeof(float), cudaMemcpyDeviceToHost, st));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->n_nnz += nnz;
-  tr->last_rows = rows;
-  return XF_OK;
+  XfBatch h{row_ptr, nullptr, labels, rows, nnz};
+  h.ids = ids;
+  return xf_step_host_batch(tr, h, 0, {XfHostReturn::NO_WAIT, nullptr, nullptr, pinned_abs_loss_sum,
+                                       "xf_trainer_step_host_ids_async"});
 }
 
 // Two-phase ingest.  _begin copies the block to the device and parses it on the trainer's ingest streams
@@ -1331,23 +1233,38 @@ static int xf_ingested_range(xf_trainer* tr, uint32_t row_start, uint32_t row_en
   return XF_OK;
 }
 
-XF_DLL int xf_trainer_step_ingested(xf_trainer* tr, uint32_t row_start, uint32_t row_end) {
+// A row slice of the current ingested block through the step kernels.  row_ptr holds absolute token offsets, so a
+// slice is just a shifted row_ptr / labels pointer.  A forward pass (mode 1) appends its predictions and labels to
+// the metric `m` and / or copies them to pctr_out / labels_out; `wait` synchronises and checks the table.
+int xf_step_ingested_slice(xf_trainer* tr, uint32_t row_start, uint32_t row_end, int mode, xf_metric* m,
+                           float* pctr_out, uint8_t* labels_out, bool wait) {
   XF_TRY(xf_ingested_range(tr, row_start, row_end));
-  if (row_end == row_start && !tr->mg) return XF_OK;
+  const uint32_t rows = row_end - row_start;
+  if (rows == 0 && !tr->mg) return XF_OK;
+  if (mode == 1 && !m && !pctr_out) return XF_ERR_ARG;
   XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
   xf_trainer::IngestSet& g = tr->ing[tr->ing_cur];
-  const uint32_t rows = row_end - row_start;
-  // row_ptr holds absolute token offsets, so a slice is just a shifted row_ptr / labels pointer; the
-  // per-token scratch (FM: touched[]) is indexed by absolute position and must not keep stale slices
-  if (!tr->table->view.lazy && !tr->mg)
-    XF_CUDA_TRY(cudaMemsetAsync(tr->touched.p, 0xFF, (size_t)tr->ing_nnz * 4, tr->table->stream));
-  XF_TRY(xf_step_device_impl(tr, g.row_ptr.as<uint32_t>() + row_start, g.keys.as<uint64_t>(),
-                             g.labels.as<uint8_t>() + row_start, rows, tr->ing_nnz, 0, nullptr));
-  XF_CUDA_TRY(cudaEventRecord(g.consumed, tr->table->stream));
-  ++tr->n_steps;
-  tr->n_rows += rows;
-  tr->last_rows = rows;
-  return XF_OK;
+  cudaStream_t st = tr->table->stream;
+  // the per-token scratch (FM: touched[]) is indexed by absolute position and must not keep stale slices
+  if (mode == 0 && !tr->table->view.lazy && !tr->mg)
+    XF_CUDA_TRY(cudaMemsetAsync(tr->touched.p, 0xFF, (size_t)tr->ing_nnz * 4, st));
+  const uint8_t* labels = g.labels.as<uint8_t>() + row_start;
+  XF_TRY(xf_step_device_impl(tr, {g.row_ptr.as<uint32_t>() + row_start, g.keys.as<uint64_t>(), labels, rows, tr->ing_nnz},
+                             mode, nullptr));
+  if (rows) {
+    if (m) XF_TRY(xf_metric_add_device(m, tr->pctr.as<float>(), labels, rows, st));
+    if (pctr_out) XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
+    if (labels_out) XF_CUDA_TRY(cudaMemcpyAsync(labels_out, labels, rows, cudaMemcpyDeviceToHost, st));
+  }
+  XF_CUDA_TRY(cudaEventRecord(g.consumed, st));
+  if (mode == 0) xf_count_step(tr, rows, 0);  // counts the slice's rows; its tokens are not counted
+  if (!wait) return XF_OK;
+  XF_CUDA_TRY(cudaStreamSynchronize(st));
+  return tr->table->check_error();
+}
+
+XF_DLL int xf_trainer_step_ingested(xf_trainer* tr, uint32_t row_start, uint32_t row_end) {
+  return xf_step_ingested_slice(tr, row_start, row_end, 0, nullptr, nullptr, nullptr, false);
 }
 
 XF_DLL int xf_trainer_ingested_export(xf_trainer* tr, uint32_t* row_ptr_out, uint64_t* keys_out, uint8_t* labels_out) {
@@ -1364,38 +1281,9 @@ XF_DLL int xf_trainer_ingested_export(xf_trainer* tr, uint32_t* row_ptr_out, uin
   return XF_OK;
 }
 
-// forward pass over a row range of the current ingested block; predictions stay in tr->pctr (metric.cu)
-int xf_trainer_forward_ingested(xf_trainer* tr, uint32_t row_start, uint32_t row_end) {
-  xf_trainer::IngestSet& g = tr->ing[tr->ing_cur];
-  return xf_step_device_impl(tr, g.row_ptr.as<uint32_t>() + row_start, g.keys.as<uint64_t>(),
-                             g.labels.as<uint8_t>() + row_start, row_end - row_start, tr->ing_nnz, 1, nullptr);
-}
-
-// Forward pass over a row range of the current block.  Asynchronous when pinned result buffers are given
-// (xf_trainer_predict_ingested_async): the caller reads them after xf_trainer_sync.
-static int xf_predict_ingested_impl(xf_trainer* tr, uint32_t row_start, uint32_t row_end, float* pctr_out,
-                                    uint8_t* labels_out, bool sync) {
-  XF_TRY(xf_ingested_range(tr, row_start, row_end));
-  if (row_end == row_start && !tr->mg) return XF_OK;
-  if (!pctr_out) return XF_ERR_ARG;
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  xf_trainer::IngestSet& g = tr->ing[tr->ing_cur];
-  const uint32_t rows = row_end - row_start;
-  cudaStream_t st = tr->table->stream;
-  XF_TRY(xf_step_device_impl(tr, g.row_ptr.as<uint32_t>() + row_start, g.keys.as<uint64_t>(),
-                             g.labels.as<uint8_t>() + row_start, rows, tr->ing_nnz, 1, nullptr));
-  if (rows) XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
-  if (labels_out && rows)
-    XF_CUDA_TRY(cudaMemcpyAsync(labels_out, g.labels.as<uint8_t>() + row_start, rows, cudaMemcpyDeviceToHost, st));
-  XF_CUDA_TRY(cudaEventRecord(g.consumed, st));
-  if (!sync) return XF_OK;
-  XF_CUDA_TRY(cudaStreamSynchronize(st));
-  return tr->table->check_error();
-}
-
 XF_DLL int xf_trainer_predict_ingested(xf_trainer* tr, uint32_t row_start, uint32_t row_end, float* pctr_out,
                                        uint8_t* labels_out) {
-  return xf_predict_ingested_impl(tr, row_start, row_end, pctr_out, labels_out, true);
+  return xf_step_ingested_slice(tr, row_start, row_end, 1, nullptr, pctr_out, labels_out, true);
 }
 
 XF_DLL int xf_trainer_set_profile(xf_trainer* tr, int on) {

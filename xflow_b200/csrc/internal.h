@@ -139,7 +139,9 @@ int xf_launch_parse(const char* d_text, uint64_t len, XfDevBuf& scratch, uint32_
                     cudaStream_t st);
 int xf_launch_hash_ids(const uint32_t* d_ids, uint32_t n, uint64_t* d_keys, cudaStream_t st);
 
-int xf_trainer_forward_ingested(xf_trainer* tr, uint32_t row_start, uint32_t row_end);  // capi.cu
+// capi.cu: train on (mode 0) or predict (mode 1) rows [row_start, row_end) of the current ingested block
+int xf_step_ingested_slice(xf_trainer* tr, uint32_t row_start, uint32_t row_end, int mode, xf_metric* m,
+                           float* pctr_out, uint8_t* labels_out, bool wait);
 
 // multi-GPU pieces implemented in comm.cu
 int xf_mg_create(xf_trainer* tr);

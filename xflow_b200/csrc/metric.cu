@@ -213,23 +213,5 @@ XF_DLL int xf_auc_logloss_device(const float* d_pctr, const uint8_t* d_labels, u
 XF_DLL int xf_trainer_predict_ingested_metric(xf_trainer* tr, uint32_t row_start, uint32_t row_end, xf_metric* m,
                                               float* pctr_out, uint8_t* labels_out) {
   if (!tr || !m) return XF_ERR_ARG;
-  if (row_start > row_end || row_end > tr->ing_rows) { xf_set_error("row range outside the ingested block"); return XF_ERR_ARG; }
-  if (tr->mg && (row_start != 0 || row_end != tr->ing_rows)) { xf_set_error("sharded trainers step whole ingested blocks"); return XF_ERR_ARG; }
-  const uint32_t rows = row_end - row_start;
-  if (rows == 0 && !tr->mg) return XF_OK;
-  XF_CUDA_TRY(cudaSetDevice(tr->table->cfg.device));
-  xf_trainer::IngestSet& g = tr->ing[tr->ing_cur];
-  cudaStream_t st = tr->table->stream;
-  XF_TRY(xf_trainer_forward_ingested(tr, row_start, row_end));
-  if (rows) {
-    XF_TRY(xf_metric_add_device(m, tr->pctr.as<float>(), g.labels.as<uint8_t>() + row_start, rows, st));
-    if (pctr_out) XF_CUDA_TRY(cudaMemcpyAsync(pctr_out, tr->pctr.p, (size_t)rows * 4, cudaMemcpyDeviceToHost, st));
-    if (labels_out) XF_CUDA_TRY(cudaMemcpyAsync(labels_out, g.labels.as<uint8_t>() + row_start, rows, cudaMemcpyDeviceToHost, st));
-  }
-  XF_CUDA_TRY(cudaEventRecord(g.consumed, st));
-  if (pctr_out || labels_out) {
-    XF_CUDA_TRY(cudaStreamSynchronize(st));
-    return tr->table->check_error();
-  }
-  return XF_OK;
+  return xf_step_ingested_slice(tr, row_start, row_end, 1, m, pctr_out, labels_out, pctr_out || labels_out);
 }
