@@ -209,11 +209,15 @@ class Table:
 
 
 class exact_sums:
-    """Context manager: accumulate the per-key gradient sums in double (analysis aid that measures the
-    float32 summation-order noise of the reference itself; NOT the reference's arithmetic)."""
+    """Context manager: accumulate the per-key gradient sums in double, and with rows=True also the per-row
+    forward sums (w x, sum v, sum v^2) (analysis aid that measures the float32 summation-order noise of the
+    reference itself; NOT the reference's arithmetic)."""
+
+    def __init__(self, rows=False):
+        self.mode = 3 if rows else 1
 
     def __enter__(self):
-        lib().xo_set_exact_sums(1)
+        lib().xo_set_exact_sums(self.mode)
 
     def __exit__(self, *a):
         lib().xo_set_exact_sums(0)

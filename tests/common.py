@@ -180,6 +180,102 @@ def check_fm_first_step(rp, keys, lab, K, v0_of, loss, export_of, alpha=0.05, be
     return uk, e
 
 
+def ftrl64(g, w, n, z, alpha=0.05, beta=1.0, l1=5e-5, l2=10.0):
+    """One FTRL-proximal step (ftrl.h:59-74) in float64."""
+    n2 = n + g * g
+    z2 = z + g - (np.sqrt(n2) - np.sqrt(n)) / alpha * w
+    w2 = np.where(np.abs(z2) <= l1, 0.0, (z2 - np.sign(z2) * l1) / -((beta + np.sqrt(n2)) / alpha + l2))
+    return w2, n2, z2
+
+
+def sigmoid64(y):
+    """Base::sigmoid (base.h:54-63) in float64: the clamps, then pow(2.718281828, y)."""
+    y = np.asarray(y, np.float64)
+    e = np.power(2.718281828, np.clip(y, -30.0, 30.0))
+    return np.where(y < -30, 1e-6, np.where(y > 30, 1.0, e / (1 + e)))
+
+
+def canonical_fm_forward64(rp, w, v, x):
+    """XF_MODEL_FM_CANONICAL's forward pass in float64, y = sum w x + 1/2 sum_k[(sum v_k x)^2 - sum (v_k x)^2],
+    on the per-token rows w[nnz], v[nnz, K] and values x[nnz].  Returns (pctr, S[B, K], row index of each token)."""
+    B = rp.size - 1
+    row_of = np.repeat(np.arange(B), np.diff(rp).astype(np.int64))
+    x64 = np.asarray(x, np.float64)
+    vx = np.asarray(v, np.float64) * x64[:, None]
+    wx = np.zeros(B); np.add.at(wx, row_of, np.asarray(w, np.float64) * x64)
+    S = np.zeros((B, vx.shape[1])); np.add.at(S, row_of, vx)
+    Q = np.zeros(B); np.add.at(Q, row_of, (vx ** 2).sum(1))
+    return sigmoid64(wx + 0.5 * ((S ** 2).sum(1) - Q)), S, row_of
+
+
+class CanonicalFM64:
+    """Float64 model of a canonical FM table trained by XF_MODEL_FM_CANONICAL (step_fmc.cu): per touched key one
+    FTRL or SGD step on w with gw = sum r x / B and on v with gv_k = (sum r x S_k - v_k sum r x^2) / B.  New keys
+    take their starting values from `pull(keys) -> (w, v)` (the table's insert-on-pull defaults)."""
+
+    FIELDS = ("w", "nw", "zw", "v", "nv", "zv")
+
+    def __init__(self, K, ftrl, pull, lr=1e-3):
+        self.K, self.ftrl, self.pull, self.lr = K, ftrl, pull, lr
+        self.state = {}
+
+    def _rows(self, keys):
+        uk, inv = np.unique(keys, return_inverse=True)
+        new = np.array([k for k in uk if int(k) not in self.state], np.uint64)
+        if new.size:
+            w0, v0 = self.pull(new)
+            for k, a, b in zip(new, w0, v0):
+                self.state[int(k)] = [float(a), 0.0, 0.0, b.astype(np.float64), np.zeros(self.K), np.zeros(self.K)]
+        W = np.array([self.state[int(k)][0] for k in uk])
+        V = np.stack([self.state[int(k)][3] for k in uk]) if uk.size else np.zeros((0, self.K))
+        return uk, inv, W, V
+
+    def forward(self, rp, keys, x):
+        uk, inv, W, V = self._rows(keys)
+        return canonical_fm_forward64(rp, W[inv], V[inv], x)[0]
+
+    def step(self, rp, keys, x, lab):
+        uk, inv, W, V = self._rows(keys)
+        B = rp.size - 1
+        p, S, row_of = canonical_fm_forward64(rp, W[inv], V[inv], x)
+        loss = p - lab
+        x64 = np.asarray(x, np.float64)
+        r = loss[row_of] * x64
+        gw = np.zeros(uk.size); np.add.at(gw, inv, r)
+        A = np.zeros((uk.size, self.K)); np.add.at(A, inv, r[:, None] * S[row_of])
+        L2 = np.zeros(uk.size); np.add.at(L2, inv, r * x64)
+        gv = (A - V * L2[:, None]) / B
+        gw = gw / B
+        for i, k in enumerate(uk):
+            s = self.state[int(k)]
+            if self.ftrl:
+                s[0], s[1], s[2] = (float(a) for a in ftrl64(gw[i], s[0], s[1], s[2]))
+                s[3], s[4], s[5] = ftrl64(gv[i], s[3], s[4], s[5])
+            else:
+                s[0] -= self.lr * gw[i]
+                s[3] = s[3] - self.lr * gv[i]
+        return loss
+
+    def export(self, keys):
+        return {f: np.array([np.atleast_1d(self.state[int(q)][j]) for q in keys]).reshape(len(keys), -1)
+                for j, f in enumerate(self.FIELDS)}
+
+
+def mvm_forward64(rp, v, fields, x):
+    """XF_MODEL_MVM's forward pass in float64, y = sum_k prod_{fields present} (sum_{tokens of the field} v_k x), on
+    the per-token rows v[nnz, K]; a row without tokens has y = 0.  Returns (pctr, S[B, 32, K], present[B, 32], row of
+    each token)."""
+    B = rp.size - 1
+    K = v.shape[1]
+    row_of = np.repeat(np.arange(B), np.diff(rp).astype(np.int64))
+    x64 = np.ones(row_of.size) if x is None else np.asarray(x, np.float64)
+    f = np.asarray(fields, np.int64)
+    S = np.zeros((B, 32, K)); np.add.at(S, (row_of, f), np.asarray(v, np.float64) * x64[:, None])
+    present = np.zeros((B, 32), bool); present[row_of, f] = True
+    y = np.where(present.any(1), np.where(present[:, :, None], S, 1.0).prod(1).sum(1), 0.0)
+    return sigmoid64(y), S, present, row_of
+
+
 def build_and_run_ps_compat(tmp_dir):
     """Compile tests/cxx/ps_compat_check.cc against the shipped headers + library and run it."""
     import subprocess

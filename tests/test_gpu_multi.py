@@ -109,9 +109,11 @@ CASES = {
     "fm_ftrl_k8": dict(model="fm", opt="ftrl", K=8, B=4096, D=32, space=200000, dist="uniform"),
     "fm_sgd_k4": dict(model="fm", opt="sgd", K=4, B=4096, D=32, space=200000, dist="uniform"),
     "fm_ftrl_k16_zipf": dict(model="fm", opt="ftrl", K=16, B=4096, D=32, space=10 ** 8, dist="zipf", edges=True),
+    "fm_ftrl_k64": dict(model="fm", opt="ftrl", K=64, B=2048, D=32, space=100000, dist="uniform"),
+    "fm_sgd_k33": dict(model="fm", opt="sgd", K=33, B=2048, D=32, space=100000, dist="uniform"),
 }
 RUNS = [(2, "lr_ftrl"), (2, "lr_ftrl_imported"), (2, "lr_ftrl_zipf_edges"), (2, "lr_sgd"), (2, "fm_ftrl_k8"), (2, "fm_sgd_k4"), (2, "fm_ftrl_k16_zipf"),
-        (4, "lr_ftrl_zipf_edges"), (4, "fm_ftrl_k16_zipf"), (8, "lr_ftrl_zipf_edges"), (8, "fm_ftrl_k16_zipf")]
+        (2, "fm_ftrl_k64"), (2, "fm_sgd_k33"), (4, "lr_ftrl_zipf_edges"), (4, "fm_ftrl_k16_zipf"), (8, "lr_ftrl_zipf_edges"), (8, "fm_ftrl_k16_zipf")]
 
 
 def _lockstep_oracle(case, world, exact):

@@ -10,8 +10,8 @@ import numpy as np
 import pytest
 
 from cases import CASES
-from common import (check_fm_first_step, assert_close, assert_close_noise_aware, data_prefixes, golden, oracle_case_run,
-                    stored_rows)
+from common import (check_fm_first_step, assert_close, assert_close_noise_aware, data_prefixes, ftrl64, golden,
+                    oracle_case_run, stored_rows)
 from oracle import oracle as O
 from xflow_b200 import api, datagen
 
@@ -495,13 +495,6 @@ def test_device_metric_matches_host_metric():
     lib.xf_metric_destroy(m)
 
 
-def _ftrl64(g, w, n, z, alpha=0.05, beta=1.0, l1=5e-5, l2=10.0):
-    n2 = n + g * g
-    z2 = z + g - (np.sqrt(n2) - np.sqrt(n)) / alpha * w
-    w2 = np.where(np.abs(z2) <= l1, 0.0, (z2 - np.sign(z2) * l1) / -((beta + np.sqrt(n2)) / alpha + l2))
-    return w2, n2, z2
-
-
 @pytest.mark.parametrize("K,opt", [(8, "ftrl"), (16, "sgd"), (4, "ftrl")])
 def test_canonical_fm_with_values_matches_float64_model(K, opt):
     """XF_MODEL_FM_CANONICAL (step_fmc.cu; SURVEY 8f-4, NOT the reference's model): the textbook FM with feature
@@ -550,8 +543,8 @@ def test_canonical_fm_with_values_matches_float64_model(K, opt):
         for i, k in enumerate(uk):
             s = state[int(k)]
             if opt == "ftrl":
-                s[0], s[1], s[2] = _ftrl64(gw[i], s[0], s[1], s[2])
-                s[3], s[4], s[5] = _ftrl64(gv[i], s[3], s[4], s[5])
+                s[0], s[1], s[2] = ftrl64(gw[i], s[0], s[1], s[2])
+                s[3], s[4], s[5] = ftrl64(gv[i], s[3], s[4], s[5])
             else:
                 s[0] -= 1e-3 * gw[i]
                 s[3] = s[3] - 1e-3 * gv[i]
@@ -620,7 +613,7 @@ def test_defined_mvm_matches_float64_model(K, opt, with_vals):
         g = A / B
         for i in np.nonzero(touched)[0]:
             if opt == "ftrl":
-                V[i], NV[i], ZV[i] = _ftrl64(g[i], V[i], NV[i], ZV[i])
+                V[i], NV[i], ZV[i] = ftrl64(g[i], V[i], NV[i], ZV[i])
             else:
                 V[i] = V[i] - lr * g[i]
     e = t.export(allk)

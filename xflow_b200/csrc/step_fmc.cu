@@ -96,7 +96,9 @@ xf_k_step_fmc(XfTableView t, const uint32_t* __restrict__ row_ptr, const uint64_
       const float rx = loss * x;
       atomicAdd(reinterpret_cast<float4*>(xf_row_ca(t, rowp)) + c, make_float4(rx * S[0], rx * S[1], rx * S[2], rx * S[3]));
       if (c == 0) {
-        const double old = atomicAdd(xf_row_g(rowp), (double)loss * (double)x);
+        // + 0.0 turns a -0.0 term (x = 0 with a negative residual) into +0.0: it must not leave the "untouched"
+        // marker in place, or a later token of the key would list the row in touched[] a second time
+        const double old = atomicAdd(xf_row_g(rowp), __dadd_rn((double)loss * (double)x, 0.0));
         atomicAdd(xf_row_acc(rowp, K), (double)loss * (double)x * (double)x);
         touched[j] = ((unsigned long long)__double_as_longlong(old) == XF_NEG_ZERO_BITS64) ? slot : XF_NO_SLOT;
       }
